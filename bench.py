@@ -2,7 +2,7 @@
 `--label_nc 35 --loadSize 2048 --n_scales_spatial 3 --use_instance --fg --use_single_G`,
 scripts/street/test_2048.sh) on synthetic 35-label sequences with random-init weights.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4|cfg2|tiny]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4|cfg2|tiny] [--dump-outputs DIR]
 
 A step = one steady-state generated frame (all three scales).  One process per GPU; N > 1 runs N
 independent clips (inference has no exchange step: "replicas only", weak scaling) and reports the
@@ -21,6 +21,12 @@ measured in the same run and reported beside it under `fast`.
                oracle/make_ref.py; CPU shims of oracle/ref_shim.py) timed on the host cores on a band of one steady-state
                frame of the same workload (kind "reference"; the oracle port, kind "port", only if no reference travelled)
 `--impl reference` times the same CPU arm as the reference line.
+
+`--dump-outputs DIR` (inference workloads) writes, for each precision mode, what the last timed step of each timed loop
+returned: `<mode>_fake_B.npy` and `<mode>_real_A.npy` from Vid2VidModelG.inference, `<mode>_e2e_rgb.npy` from
+inference_stream (the uint8 frame as float32), all on the same fixed seeded sample of DUMP_PIXELS pixel positions
+(`sample_pixels.npy`), channels first.  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -151,12 +157,14 @@ def peaks():
 
 # ----------------------------------------------------------------------------------------------- ours
 MODES = ('precise', 'fast')
+DUMP_PIXELS = 1 << 17       # per mode 3 + 36 + 3 float32 channels at these positions: 2 modes * 42 * 4 B * 2^17 = 44 MB
 DTYPE = {'precise': 'bf16x3 (split-bf16 hi/lo operands, 3 tcgen05.mma per K block, fp32 accumulate: fp32-class)',
          'fast': 'bf16 (bf16 operands, fp32 accumulate)'}
 
 
 def run_ours(args, rank, world, local_rank):
     import gc
+    import numpy as np
     import torch
     import torch.distributed as dist
     from vid2vid_b200 import _lib as L
@@ -186,6 +194,11 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
 
     modes = [m for m in MODES if args.modes in ('both', m)]
+    dumps = {}
+    if args.dump_outputs:
+        pix = torch.randperm(H * Wd, generator=torch.Generator().manual_seed(0))[:DUMP_PIXELS].sort().values
+        pix_dev = pix.to(dev)
+        dumps['sample_pixels'] = pix.double()
     sampler = ClockSampler(local_rank)
     sampler.start()
     res = {}
@@ -210,10 +223,13 @@ def run_ours(args, rank, world, local_rank):
         e0.record()
         for _ in range(K):
             A = seq_dev[:, t:t + tG]
-            model.inference(A, None, A)
+            out = model.inference(A, None, A)
             t += 1
         e1.record()
         barrier()
+        if args.dump_outputs:       # (the next inference call may reuse these buffers)
+            dumps[mode + '_fake_B'] = out[0][0].flatten(1)[:, pix_dev].cpu()
+            dumps[mode + '_real_A'] = out[1].flatten(1)[:, pix_dev].cpu()
         ms_dev = e0.elapsed_time(e1)
         launches = L.LAUNCHES[0] - l0
         # ---- timed: end to end through the public streaming API with HOST buffers: one pinned uint8 label frame (and the
@@ -230,6 +246,8 @@ def run_ours(args, rank, world, local_rank):
             t += 1
         e3.record()
         barrier()
+        if args.dump_outputs:
+            dumps[mode + '_e2e_rgb'] = out_u8.view(-1, 3)[pix].t().float()
         gc.enable()
         ms_e2e = e2.elapsed_time(e3)
         ms_dev, ms_e2e = reduce_times([ms_dev, ms_e2e], world, dev)
@@ -239,6 +257,11 @@ def run_ours(args, rank, world, local_rank):
     d2h = 3 * H * Wd             # uint8 RGB frame
     if rank != 0:
         return
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            a = a.numpy()
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a if a.dtype == np.float64 else a.astype(np.float32))
 
     # ---- first-frame generator (--use_single_G; runs tG - 1 times per clip, not per frame): timed separately (SURVEY 8d)
     first_ms = None
@@ -656,7 +679,11 @@ def main():
     ap.add_argument('--workload', default='cfg4', choices=list(WORKLOADS))
     ap.add_argument('--no-cpu-baseline', dest='no_cpu_baseline', action='store_true')
     ap.add_argument('--modes', default='both', choices=['both', 'precise', 'fast'])
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (inference workloads)')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'ours' or WORKLOADS[args.workload].get('train') or WORKLOADS[args.workload].get('flownet')):
+        ap.error('--dump-outputs is implemented for --impl ours on the inference workloads (cfg4, cfg2, tiny)')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

@@ -1,19 +1,17 @@
 """Pins oracle/flownet2_oracle.py (SURVEY 8 rows a14 / a15: the reference flow network behind the training targets).
-  * against the unmodified reference modules (models/flownet2_pytorch/models.py, models/flownet.py) when /root/reference
-    is present -- the three native ops are CUDA-only there and are supplied by oracle/flowops_oracle.c on both sides,
-    so this pins the network wiring, layer hyper-parameters and the wrapper logic, not those ops;
-  * against the committed fixture tests/golden/flownet2_small.npz (reference output on seeded inputs with weights
-    regenerated from (seed, key, shape)) everywhere else.  CPU only."""
+  * against the committed fixtures tests/golden/flownet2_small.npz and flownet2_pins.npz: outputs of the unmodified
+    reference modules (models/flownet2_pytorch/models.py, models/flownet.py) on seeded inputs, with weights regenerated
+    from (seed, key, shape).  The three native ops are CUDA-only in the reference and were supplied by
+    oracle/flowops_oracle.c there, so this pins the network wiring, layer hyper-parameters and the wrapper logic, not
+    those ops.  CPU only."""
 import json
 import os
-import types
 
 import numpy as np
-import pytest
 import torch
 
+import cases
 from oracle import flownet2_oracle as FO
-from oracle import ref_shim
 
 GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
@@ -40,36 +38,21 @@ def test_flownet2_oracle_vs_golden():
     assert float(np.abs(wconf.numpy() - g['wconf']).mean()) < 2e-3
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='reference tree not present (GPU box)')
 def test_flownet2_oracle_vs_reference_random_init():
-    F2 = ref_shim.flownet2_class()
-    torch.manual_seed(3)
-    net = F2().eval()                                   # the reference's own Xavier / uniform-bias initialisation
-    sd = net.state_dict()
-    pair = torch.rand(2, 3, 2, 64, 64)
+    keys = json.load(open(os.path.join(GOLD, 'flownet2_keys.json')))
+    sd = FO.det_state_dict(keys, seed=3)
+    g = np.load(os.path.join(GOLD, 'flownet2_pins.npz'))
+    i = cases.flownet2_pin_inputs()
     with torch.no_grad():
-        ref = net(pair)
-        out = FO.flownet2(sd, pair)
-    _close(out, ref, 'FlowNet2 (batch 2, 64x64)')
-    # sub-networks on their own inputs (eval mode returns a 1-tuple)
-    x6, x12 = torch.rand(1, 6, 64, 128) - 0.5, torch.rand(1, 12, 64, 128) - 0.5
-    with torch.no_grad():
-        _close(FO.flownet_c(sd, 'flownetc.', x6), net.flownetc(x6)[0], 'FlowNetC')
-        _close(FO.flownet_s(sd, 'flownets_1.', x12), net.flownets_1(x12)[0], 'FlowNetS')
-        _close(FO.flownet_sd(sd, 'flownets_d.', x6), net.flownets_d(x6)[0], 'FlowNetSD')
-    xf = torch.rand(1, 11, 64, 64, generator=torch.Generator().manual_seed(1))
-    with torch.no_grad():
-        _close(FO.flownet_fusion(sd, 'flownetfusion.', xf), net.flownetfusion(xf), 'FlowNetFusion')
+        _close(FO.flownet2(sd, i['pair']), g['flow'], 'FlowNet2 (batch 2, 64x64)')
+        # sub-networks on their own inputs (eval mode returns a 1-tuple)
+        _close(FO.flownet_c(sd, 'flownetc.', i['x6']), g['flownetc'], 'FlowNetC')
+        _close(FO.flownet_s(sd, 'flownets_1.', i['x12']), g['flownets_1'], 'FlowNetS')
+        _close(FO.flownet_sd(sd, 'flownets_d.', i['x6']), g['flownets_d'], 'FlowNetSD')
+        _close(FO.flownet_fusion(sd, 'flownetfusion.', i['xf']), g['flownetfusion'], 'FlowNetFusion')
     # the vid2vid wrapper (models/flownet.py:43-58), un-resized and resized paths
-    from models.flownet import FlowNet                                                        # noqa (reference module)
-    from models.flownet2_pytorch.networks.resample2d_package.resample2d import Resample2d     # noqa
-    stub = types.SimpleNamespace(flowNet=net, resample=Resample2d())
-    stub.norm = lambda t: FlowNet.norm(stub, t)
-    for h, w in ((64, 64), (70, 64)):
-        im1 = torch.rand(1, 3, h, w)
-        im2 = torch.roll(im1, shifts=(1, 1), dims=(2, 3))
+    for h, w in cases.FLOWNET2_PIN_SIZES:
         with torch.no_grad():
-            rf, rc = FlowNet.compute_flow_and_conf(stub, im1, im2)
-            of, oc = FO.flow_and_conf(sd, im1, im2)
-        _close(of, rf, 'wrapper flow %dx%d' % (h, w))
-        assert float((oc - rc).abs().mean()) < 2e-3
+            of, oc = FO.flow_and_conf(sd, i['im1_%d' % h], i['im2_%d' % h])
+        _close(of, g['wflow_%d' % h], 'wrapper flow %dx%d' % (h, w))
+        assert float(np.abs(oc.numpy() - g['wconf_%d' % h]).mean()) < 2e-3

@@ -12,7 +12,6 @@ from oracle.make_golden import coarse_feats
 from vid2vid_b200.utils import det_fill_, synth_label_sequence
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 # Stated tolerances against the fp32 reference (DESIGN.md 4), (max |d|, mean |d|); images and masks live in [-1,1] / [0,1],
 # features are O(1) (rms ~0.7), flow is in pixels and carries the x20*2^s head scale.
@@ -41,7 +40,7 @@ def mode(request):
 
 
 def load(name):
-    return dict(np.load(os.path.join(GOLD, name + '.npz')))
+    return C.load_golden(name)
 
 
 def report(name, key, out, gold):

@@ -1,6 +1,5 @@
 """GPU parity of Vid2VidModelG.inference (multi-scale, --fg --use_single_G) against the reference fixture
 and the oracle driver."""
-import os
 
 import numpy as np
 import pytest
@@ -12,7 +11,6 @@ from vid2vid_b200.model_g import Vid2VidModelG
 from vid2vid_b200.utils import det_fill_, synth_label_sequence
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 
 @pytest.mark.parametrize('mode', ['precise', 'fast'])
@@ -29,7 +27,7 @@ def _inference_sequence(mode):
     c = C.CASES['infer_s3']
     opt = C.inference_opt(c)
     opt.gpu_ids = [0]
-    gold = dict(np.load(os.path.join(GOLD, 'infer_s3.npz')))
+    gold = C.load_golden('infer_s3')
     m = Vid2VidModelG()
     m.use_single_G = False
     opt.use_single_G = False               # build without touching checkpoints/, then attach the seeded nets

@@ -1,22 +1,17 @@
-"""CPU: the host-side checkpoint / schedule helpers (vid2vid_b200/base_model.py) against the reference's BaseModel
-(models/base_model.py:43-48,154-181) run on the same state."""
+"""CPU: the host-side checkpoint / schedule helpers (vid2vid_b200/base_model.py) against what the reference's BaseModel
+(models/base_model.py:43-48,154-181) did on the same state (tests/golden/base_model_schedule.json, written by
+`python -m oracle.make_golden schedule`)."""
+import json
 import os
 import types
 
-import pytest
 import torch
 import torch.nn as nn
 
+import cases
 from vid2vid_b200.base_model import HostScheduleMixin
 
-
-def _ref_base_model():
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip('reference tree not available')
-    ref_shim.install()
-    from models.base_model import BaseModel
-    return BaseModel
+REF = json.load(open(os.path.join(os.path.dirname(__file__), 'golden', 'base_model_schedule.json')))
 
 
 class _Ours(HostScheduleMixin):
@@ -36,45 +31,33 @@ def _state(opt, cls):
 
 
 def _opt(tmp):
-    return types.SimpleNamespace(checkpoints_dir=str(tmp), name='run', lr=2e-4, niter=10, niter_decay=10, beta1=0.5,
-                                 max_frames_backpropagate=4, max_frames_per_gpu=8)
+    return types.SimpleNamespace(checkpoints_dir=str(tmp), **cases.SCHEDULE_OPT)
 
 
 def test_schedules_match_the_reference(tmp_path):
-    Ref = _ref_base_model()
     opt = _opt(tmp_path)
-    ours, ref = _state(opt, _Ours), _state(opt, Ref)
-    ref.save_dir = os.path.join(opt.checkpoints_dir, opt.name)
-    for epoch in (11, 15, 20):
+    ours = _state(opt, _Ours)
+    for epoch, (old_lr, lrs) in zip(cases.SCHEDULE_EPOCHS, REF['lr'], strict=True):
         ours.update_learning_rate(epoch, 'G')
-        ref.update_learning_rate(epoch, 'G')
-        assert ours.old_lr == ref.old_lr
-        assert [g['lr'] for g in ours.optimizer_G.param_groups] == [g['lr'] for g in ref.optimizer_G.param_groups]
-    for ratio in range(1, 6):                                   # train.py:121-123: every niter_step epochs
+        assert ours.old_lr == old_lr
+        assert [g['lr'] for g in ours.optimizer_G.param_groups] == lrs
+    for ratio, batch in zip(cases.SCHEDULE_RATIOS, REF['batch'], strict=True):     # train.py:121-123: every niter_step epochs
         ours.update_training_batch(ratio)
-        ref.update_training_batch(ratio)
-        assert (ours.n_frames_bp, ours.n_frames_per_gpu, ours.n_frames_load) == (ref.n_frames_bp, ref.n_frames_per_gpu, ref.n_frames_load)
+        assert [ours.n_frames_bp, ours.n_frames_per_gpu, ours.n_frames_load] == batch
     assert ours.n_frames_per_gpu == 8
     ours.update_fixed_params()
-    ref.update_fixed_params()
-    assert ours.finetune_all and ref.finetune_all
+    assert ours.finetune_all and REF['finetune_all']
     n_ours = sum(p.numel() for g in ours.optimizer_G.param_groups for p in g['params'])
-    n_ref = sum(p.numel() for g in ref.optimizer_G.param_groups for p in g['params'])
-    assert n_ours == n_ref == sum(p.numel() for m in (ours.netG0, ours.netG1) for p in m.parameters())
-    assert ours.optimizer_G.param_groups[0]['lr'] == ref.optimizer_G.param_groups[0]['lr'] == ours.old_lr
+    assert n_ours == REF['n_params_G'] == sum(p.numel() for m in (ours.netG0, ours.netG1) for p in m.parameters())
+    assert ours.optimizer_G.param_groups[0]['lr'] == REF['lr_after_fix'] == ours.old_lr
 
 
 def test_save_network_writes_the_reference_file_and_keeps_the_parameters_in_place(tmp_path):
-    Ref = _ref_base_model()
     opt = _opt(tmp_path)
-    ours, ref = _state(opt, _Ours), _state(opt, Ref)
-    ref.save_dir = os.path.join(opt.checkpoints_dir, 'ref')
-    os.makedirs(ref.save_dir)
-    ref.netG1.load_state_dict(ours.netG1.state_dict())
+    ours = _state(opt, _Ours)
     ptrs = [p.data_ptr() for p in ours.netG1.parameters()]
     path = ours.save_network(ours.netG1, 'G1', 'latest', [])
-    ref.save_network(ref.netG1, 'G1', 'latest', [])
-    assert os.path.basename(path) == 'latest_net_G1.pth' and os.path.dirname(path) == os.path.join(opt.checkpoints_dir, opt.name)
-    a, b = torch.load(path), torch.load(os.path.join(ref.save_dir, 'latest_net_G1.pth'))
-    assert list(a) == list(b) and all(torch.equal(a[k], b[k]) and a[k].device.type == 'cpu' for k in a)
+    assert [os.path.basename(path)] == REF['saved_files'] and os.path.dirname(path) == os.path.join(opt.checkpoints_dir, opt.name)
+    a, b = torch.load(path), ours.netG1.state_dict()
+    assert list(a) == REF['saved_keys'] and all(torch.equal(a[k], b[k]) and a[k].device.type == 'cpu' for k in a)
     assert ptrs == [p.data_ptr() for p in ours.netG1.parameters()]          # no .cpu() / .cuda() round trip of the module

@@ -1,52 +1,40 @@
 """Pins oracle/losses_oracle.py (SURVEY 8 row a13: warp / flow / GAN / feature-matching losses of the training step)
-against the unmodified reference Vid2VidModelD.forward (models/vid2vid_model_D.py:92-197) on CPU, --no_vgg.
-Needs /root/reference (build container); skipped on the GPU box."""
+against the unmodified reference Vid2VidModelD.forward (models/vid2vid_model_D.py:92-197) on CPU, --no_vgg, through its
+outputs on seeded inputs (tests/golden/ref_losses.npz, written by `python -m oracle.make_golden losses`)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
+import cases
 from oracle import losses_oracle as LO
-from oracle import ref_shim
-from vid2vid_b200.utils import make_opt
+from vid2vid_b200 import networks as NW
+from vid2vid_b200.utils import det_fill_
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason='reference tree not present (GPU box)')
-
-
-def _model(**kw):
-    ref_shim.install()
-    from models.vid2vid_model_D import Vid2VidModelD          # noqa (reference module)
-    opt = make_opt(label_nc=35, use_instance=True, isTrain=True, gpu_ids=[0], n_gpus_gen=1, no_vgg=True, **kw)
-    opt.add_face_disc = False
-    opt.debug = True
-    opt.load_pretrain = ''
-    torch.manual_seed(5)
-    m = Vid2VidModelD()
-    m.initialize(opt)
-    return m, opt
+GOLD = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'ref_losses.npz'))
 
 
-def _rand(shape, g, lo=-1.0, hi=1.0):
-    return torch.rand(shape, generator=g) * (hi - lo) + lo
+def _netD_sd(opt, input_nc, seed):
+    """The discriminator Vid2VidModelD.initialize builds (vid2vid_model_D.py:28-38), filled as the pins fill the reference's."""
+    return det_fill_(NW.define_D(input_nc, opt.ndf, opt.n_layers_D, opt.norm, opt.num_D, not opt.no_ganFeat, []), seed=seed).state_dict()
+
+
+def _ref(key, n):
+    return [torch.from_numpy(GOLD['%s_%d' % (key, i)]) for i in range(n)]
 
 
 @pytest.mark.parametrize('no_first_img,with_raw', [(False, True), (True, False)])
 def test_spatial_losses_match_reference(no_first_img, with_raw):
-    m, opt = _model(n_scales_spatial=2, no_first_img=no_first_img)
-    g = torch.Generator().manual_seed(1)
-    h, w = 48, 64
-    real_B, fake_B, real_B_prev, fake_B_prev = (_rand((1, 3, h, w), g) for _ in range(4))
-    fake_B_raw = _rand((1, 3, h, w), g) if with_raw else None
-    real_A = (_rand((1, 36, h, w), g) > 0.8).float()
-    flow, flow_ref = _rand((1, 2, h, w), g, -3, 3), _rand((1, 2, h, w), g, -3, 3)
-    weight = _rand((1, 1, h, w), g, 0, 1)
-    conf = (_rand((1, 1, h, w), g) > 0).float()
+    opt = cases.pin_loss_opt(n_scales_spatial=2, no_first_img=no_first_img)
+    sd = _netD_sd(opt, opt.label_nc + 1 + opt.output_nc, cases.PIN_SEED_D)
     with torch.no_grad():
-        ref = m.forward(0, [real_B, fake_B, fake_B_raw, real_A, real_B_prev, fake_B_prev, flow, weight, flow_ref, conf])
-        ours = LO.spatial_losses(m.netD.state_dict(), real_B, fake_B, fake_B_raw, real_A, real_B_prev, fake_B_prev, flow, weight,
-                                 flow_ref, conf, lambda_F=opt.lambda_F, lambda_T=opt.lambda_T, lambda_feat=opt.lambda_feat,
-                                 n_scales_spatial=opt.n_scales_spatial, no_first_img=no_first_img, num_D=opt.num_D,
-                                 n_layers_D=opt.n_layers_D, norm=opt.norm)
+        ours = LO.spatial_losses(sd, *cases.pin_spatial_loss_inputs(with_raw), lambda_F=opt.lambda_F, lambda_T=opt.lambda_T,
+                                 lambda_feat=opt.lambda_feat, n_scales_spatial=opt.n_scales_spatial, no_first_img=no_first_img,
+                                 num_D=opt.num_D, n_layers_D=opt.n_layers_D, norm=opt.norm)
     names = ['G_VGG', 'G_GAN', 'G_GAN_Feat', 'D_real', 'D_fake', 'G_Warp', 'F_Flow', 'F_Warp', 'W']
-    assert len(ref) == len(ours) == len(names)
+    ref = _ref('spatial_%d' % no_first_img, len(names))
+    assert len(ours) == len(names)
     for n, a, b in zip(names, ours, ref):
         # (G_VGG under --no_vgg and W without --no_first_img are zeros_like(weight): H*W rows of zeros in both)
         assert a.shape == b.shape, (n, a.shape, b.shape)
@@ -56,15 +44,13 @@ def test_spatial_losses_match_reference(no_first_img, with_raw):
 
 
 def test_temporal_losses_match_reference():
-    m, opt = _model()
-    g = torch.Generator().manual_seed(2)
-    h, w, tD = 48, 64, opt.n_frames_D
-    real_B, fake_B = _rand((1, tD, 3, h, w), g), _rand((1, tD, 3, h, w), g)
-    flow_ref = _rand((1, tD - 1, 2, h, w), g, -40, 40)
-    conf = (_rand((1, tD - 1, 1, h, w), g) > 0).float()
+    opt = cases.pin_loss_opt()
+    tD = opt.n_frames_D
+    sd = _netD_sd(opt, opt.output_nc * tD + 2 * (tD - 1), cases.PIN_SEED_D_T)
     with torch.no_grad():
-        ref = m.forward(1, [real_B, fake_B, flow_ref, conf])
-        ours = LO.temporal_losses(m.netD_T0.state_dict(), real_B, fake_B, flow_ref, conf, n_frames_D=tD, output_nc=3,
+        ours = LO.temporal_losses(sd, *cases.pin_temporal_loss_inputs(opt), n_frames_D=tD, output_nc=3,
                                   lambda_feat=opt.lambda_feat, num_D=opt.num_D, n_layers_D=opt.n_layers_D, norm=opt.norm)
-    for n, a, b in zip(['G_T_GAN', 'G_T_GAN_Feat', 'D_T_real', 'D_T_fake', 'G_T_Warp'], ours, ref):
+    names = ['G_T_GAN', 'G_T_GAN_Feat', 'D_T_real', 'D_T_fake', 'G_T_Warp']
+    assert len(ours) == len(names)
+    for n, a, b in zip(names, ours, _ref('temporal', len(names))):
         assert torch.allclose(a, b, rtol=1e-4, atol=1e-6), (n, float(a), float(b))

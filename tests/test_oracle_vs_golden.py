@@ -1,6 +1,5 @@
 """Pins oracle/generator_oracle.py against the committed fixtures (outputs of the unmodified
 reference, oracle/make_golden.py).  CPU-only; this is the check that travels to the GPU box."""
-import os
 
 import numpy as np
 import pytest
@@ -12,17 +11,18 @@ from oracle.make_golden import coarse_feats
 from vid2vid_b200.utils import det_fill_, synth_label_sequence
 from vid2vid_b200 import networks as NW
 
-GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 
 def load(name):
-    return dict(np.load(os.path.join(GOLD, name + '.npz')))
+    return C.load_golden(name)
 
 
 def close(a, gold, tol=3e-5):
     a = a.detach().numpy()
     assert a.shape == gold.shape, (a.shape, gold.shape)
-    assert np.abs(a - gold).max() <= tol, np.abs(a - gold).max()
+    # relative to the output's magnitude where it exceeds 1 (flow is in pixels, x20 head scale): the CPU convolutions sum in
+    # an order that depends on the host's vector ISA and thread count (3.3e-5 on flows of ~8 px seen between two hosts)
+    assert np.abs(a - gold).max() <= tol * max(1.0, float(np.abs(gold).max())), np.abs(a - gold).max()
 
 
 def build_state_dict(c):
