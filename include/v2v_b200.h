@@ -116,6 +116,22 @@ int v2v_avgpool3s2_backward(const float* grad_out, float* grad_in, int P, int H,
 int v2v_resample_backward(const float* image, const float* flow, const float* grad_out, float* grad_image, float* grad_flow, int N,
                           int C, int H, int W, int align_corners, v2v_stream_t stream);
 
+/* Face discriminator of the pose training step (--add_face_disc, models/vid2vid_model_D.py:148-158,215-230).
+ * face_window: bounding box, over all N images of real_A (N,C,H,W), of the face pixels -- channel 2 > 0.9 (predicate 0) or, with
+ *   --openpose_only (predicate 1), 0.19 < c0 < 0.21 && c1 < -0.99 && -0.61 < c2 < -0.59, compared in fp32 -- turned into the
+ *   reference's fixed window: centre clamped to [half, dim - 1 - half], window [centre - half, centre + half) per axis.
+ *   win: 10 int32 of device memory, zeroed by the caller before the first call and reusable afterwards (one launch per call,
+ *   no memset): win[0..4] = {found, ys, ye, xs, xe} (all 0 when no face pixel exists), win[5..9] scratch left zeroed.
+ * crop_concat_forward: out (N, Ca+Cb, Ly, Lx) = cat(a[:, :, ys:ys+Ly, xs:xs+Lx], b[...same window...], dim=1), a (N,Ca,H,W),
+ *   b (N,Cb,H,W), the window origin read from win[1] / win[3] on the device.
+ * crop_backward: grad_b (N,Cb,H,W) = channels [c_off, c_off+Cb) of grad_out (N, c_off+Cb, Ly, Lx) inside the window, 0 outside. */
+int v2v_face_window(const float* real_A, int N, int C, int H, int W, int predicate, int half_y, int half_x, int32_t* win,
+                    v2v_stream_t stream);
+int v2v_crop_concat_forward(const float* a, int Ca, const float* b, int Cb, int N, int H, int W, const int32_t* win, int Ly, int Lx,
+                            float* out, v2v_stream_t stream);
+int v2v_crop_backward(const float* grad_out, int c_off, int Cb, int N, int H, int W, const int32_t* win, int Ly, int Lx, float* grad_b,
+                      v2v_stream_t stream);
+
 /* FlowNet2 glue (models/flownet2_pytorch/models.py:97-160, models/flownet.py:43-58), fp32 NCHW.
  * flownet_prep: the image pair -> x (B,6,H,W) = (pair - mean over both frames and all pixels, per sample and colour) / rgb_max,
  *   frame 0 in channels 0-2, frame 1 in 3-5 (models.py:97-103); x1 (may be NULL) = the frame-1 half as its own contiguous

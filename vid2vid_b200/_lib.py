@@ -41,6 +41,7 @@ SYMBOLS = [
     'v2v_version', 'v2v_last_error',
     'v2v_correlation_out_shape', 'v2v_correlation_forward', 'v2v_resample2d_forward', 'v2v_channelnorm_forward',
     'v2v_resample_forward', 'v2v_onehot_edges', 'v2v_avgpool3s2', 'v2v_fg_mask',
+    'v2v_face_window', 'v2v_crop_concat_forward', 'v2v_crop_backward',
     'v2v_l1_loss_forward', 'v2v_l1_loss_backward', 'v2v_mse_const_forward', 'v2v_mse_const_backward', 'v2v_avgpool3s2_backward',
     'v2v_resample_backward', 'v2v_ids_window_push', 'v2v_tensor2im_u8', 'v2v_flownet_prep', 'v2v_resize', 'v2v_sub_channels', 'v2v_flow_conf',
     'v2v_plan_create', 'v2v_plan_destroy', 'v2v_plan_set_precision', 'v2v_g_input', 'v2v_g_input_ex', 'v2v_g_conv', 'v2v_g_norm_act', 'v2v_g_norm_act_slice', 'v2v_g_conv_act',
@@ -107,6 +108,9 @@ def lib():
     l.v2v_mse_const_backward.argtypes = [fp, C.c_int64, C.c_float, fp, fp, vp]
     l.v2v_avgpool3s2_backward.argtypes = [fp, fp, C.c_int, C.c_int, C.c_int, vp]
     l.v2v_resample_backward.argtypes = [fp, fp, fp, fp, fp] + [C.c_int] * 5 + [vp]
+    l.v2v_face_window.argtypes = [fp] + [C.c_int] * 7 + [vp, vp]
+    l.v2v_crop_concat_forward.argtypes = [fp, C.c_int, fp] + [C.c_int] * 4 + [vp, C.c_int, C.c_int, fp, vp]
+    l.v2v_crop_backward.argtypes = [fp] + [C.c_int] * 5 + [vp, C.c_int, C.c_int, fp, vp]
     l.v2v_ids_window_push.argtypes = [fp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     l.v2v_tensor2im_u8.argtypes = [fp, vp, C.c_int, C.c_int, C.c_int, vp]
     l.v2v_flownet_prep.argtypes = [fp, fp, C.c_int64, C.c_int64, fp, fp, fp, C.c_int, C.c_int, C.c_int, C.c_float, vp]

@@ -5,7 +5,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
-SOURCES = ['conv_umma.cu', 'conv_simt.cu', 'norm.cu', 'layout.cu', 'warp.cu', 'pyramid.cu', 'flowops.cu', 'flownet_glue.cu', 'backward.cu', 'wgrad_umma.cu', 'losses.cu', 'plan.cu',
+SOURCES = ['conv_umma.cu', 'conv_simt.cu', 'norm.cu', 'layout.cu', 'warp.cu', 'pyramid.cu', 'flowops.cu', 'flownet_glue.cu', 'backward.cu', 'wgrad_umma.cu', 'losses.cu', 'face.cu', 'plan.cu',
            'api.cu']
 LIB = os.path.join(HERE, 'libv2v_b200.so')
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')

@@ -28,6 +28,9 @@ cudaError_t launch_avgpool3s2_bwd(const float*, float*, int, int, int, cudaStrea
 cudaError_t launch_resample_bwd(const float*, const float*, const float*, float*, float*, int, int, int, int, int, cudaStream_t);
 struct FgLabels { int v[16]; };
 cudaError_t launch_fg_mask(const float*, float*, int, int, int, int, int, int, FgLabels, int, cudaStream_t);
+cudaError_t launch_face_window(const float*, int, int, int, int, int, int, int, int*, cudaStream_t);
+cudaError_t launch_crop_concat(const float*, int, const float*, int, int, int, int, const int*, int, int, float*, cudaStream_t);
+cudaError_t launch_crop_backward(const float*, int, int, int, int, int, const int*, int, int, float*, cudaStream_t);
 }  // namespace v2v
 
 using namespace v2v;
@@ -120,6 +123,32 @@ int v2v_fg_mask(const float* real_A, float* mask, int B, int T, int C, int H, in
     l.v[i] = fg_labels[i];
   }
   API_CUDA(launch_fg_mask(real_A, mask, B, T, C, H, W, t, l, n_labels, reinterpret_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
+int v2v_face_window(const float* real_A, int N, int C, int H, int W, int predicate, int half_y, int half_x, int32_t* win,
+                    v2v_stream_t stream) {
+  API_REQUIRE(real_A && win && N > 0 && C >= 3 && H > 0 && W > 0, "face_window: bad arguments");
+  API_REQUIRE(predicate == 0 || predicate == 1, "face_window: predicate %d unknown", predicate);
+  API_REQUIRE(half_y >= 0 && half_x >= 0 && 2 * half_y <= H && 2 * half_x <= W,
+              "face_window: %dx%d window larger than the %dx%d frame", 2 * half_y, 2 * half_x, H, W);
+  API_CUDA(launch_face_window(real_A, N, C, H, W, predicate, half_y, half_x, win, reinterpret_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
+int v2v_crop_concat_forward(const float* a, int Ca, const float* b, int Cb, int N, int H, int W, const int32_t* win, int Ly, int Lx,
+                            float* out, v2v_stream_t stream) {
+  API_REQUIRE(a && b && win && out && Ca > 0 && Cb > 0 && N > 0, "crop_concat_forward: bad arguments");
+  API_REQUIRE(Ly > 0 && Lx > 0 && Ly <= H && Lx <= W, "crop_concat_forward: %dx%d window outside the %dx%d frame", Ly, Lx, H, W);
+  API_CUDA(launch_crop_concat(a, Ca, b, Cb, N, H, W, win, Ly, Lx, out, reinterpret_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
+int v2v_crop_backward(const float* grad_out, int c_off, int Cb, int N, int H, int W, const int32_t* win, int Ly, int Lx, float* grad_b,
+                      v2v_stream_t stream) {
+  API_REQUIRE(grad_out && win && grad_b && c_off >= 0 && Cb > 0 && N > 0, "crop_backward: bad arguments");
+  API_REQUIRE(Ly > 0 && Lx > 0 && Ly <= H && Lx <= W, "crop_backward: %dx%d window outside the %dx%d frame", Ly, Lx, H, W);
+  API_CUDA(launch_crop_backward(grad_out, c_off, Cb, N, H, W, win, Ly, Lx, grad_b, reinterpret_cast<cudaStream_t>(stream)));
   return 0;
 }
 

@@ -4,6 +4,7 @@ operator surface (same class names / argument meaning / output-ownership rules):
   Correlation / Resample2d / ChannelNorm  <- models/flownet2_pytorch/networks/*_package/*.py
   resample(image, flow)                   <- BaseModel.resample (models/base_model.py:189-196)
   onehot_edges / avgpool3s2 / fg_mask     <- Vid2VidModelG.encode_input / build_pyr / compute_mask
+  face_window / crop_concat               <- Vid2VidModelD.get_face_region + the face crop (--add_face_disc)
 
 CUDA fp32 contiguous tensors only; errors from the library raise RuntimeError (the reference's
 wrapper raises via AT_ERROR, correlation_cuda.cc:81-83).  No CPU fallback.
@@ -275,3 +276,82 @@ class MseConstFunction(torch.autograd.Function):
 
 def mse_to_const(x, target):
     return MseConstFunction.apply(x, target)
+
+
+# ------------------------------------------------------------------------------------------------ face discriminator
+FACE_WINDOW_WORDS = 10      # {found, ys, ye, xs, xe} + the kernel's accumulators (include/v2v_b200.h)
+
+
+def face_window_buffer(device):
+    """Device buffer for face_window(..., buf=): zeroed once here, left reusable by every call."""
+    return torch.zeros(FACE_WINDOW_WORDS, device=device, dtype=torch.int32)
+
+
+def face_half(fine_size):
+    """Half the side of the face window: the reference's fineSize // 32 * 8 (vid2vid_model_D.py:224-225) halved."""
+    return fine_size // 32 * 8 // 2
+
+
+def face_window(real_A, fine_size, openpose_only=False, buf=None):
+    """Vid2VidModelD.get_face_region (vid2vid_model_D.py:215-230) on the device: real_A (N, C, H, W) -> int32 tensor
+    {found, ys, ye, xs, xe} (all zero when no face pixel exists).  One launch, no host synchronisation; `buf` (from
+    face_window_buffer) avoids allocating and zeroing a buffer per call, and the result is a view into it."""
+    real_A = real_A.contiguous()
+    _chk(real_A)
+    n, c, h, w = real_A.shape
+    half = face_half(fine_size)
+    if c < 3:
+        raise ValueError('face_window needs at least 3 input channels, got %d' % c)
+    if 2 * half > h or 2 * half > w:
+        raise ValueError('face window %dx%d (fineSize %d) is larger than the %dx%d frame' % (2 * half, 2 * half, fine_size, h, w))
+    if buf is None:
+        buf = face_window_buffer(real_A.device)
+    if buf.dtype != torch.int32 or buf.device != real_A.device or buf.numel() != FACE_WINDOW_WORDS or not buf.is_contiguous():
+        raise RuntimeError('face_window: buf must be a contiguous int32 tensor of %d words on the input device' % FACE_WINDOW_WORDS)
+    with _on(real_A):
+        _ck(L.lib().v2v_face_window(_p(real_A), n, c, h, w, int(bool(openpose_only)), half, half, _p(buf), _st(real_A)))
+    return buf[:5]
+
+
+def _chk_win(win, dev):
+    if win.dtype != torch.int32 or win.device != dev or win.numel() < 5 or not win.is_contiguous():
+        raise RuntimeError('crop window must be a contiguous int32 device tensor {found, ys, ye, xs, xe}')
+
+
+class CropConcatFunction(torch.autograd.Function):
+    """cat(a[:, :, ys:ys+L, xs:xs+L], b[..same..], dim=1) with the window read on the device; the gradient goes to b only
+    (a is the condition real_A, which needs none)."""
+
+    @staticmethod
+    def forward(ctx, a, b, win, size):
+        a, b = a.detach().contiguous(), b.detach().contiguous()
+        _chk(a, b)
+        _chk_win(win, a.device)
+        n, ca, h, w = a.shape
+        cb = b.shape[1]
+        if b.shape[0] != n or tuple(b.shape[2:]) != (h, w):
+            raise RuntimeError('crop_concat: a %s and b %s differ in batch or frame size' % (tuple(a.shape), tuple(b.shape)))
+        if size > h or size > w:
+            raise ValueError('crop window %dx%d is larger than the %dx%d frame' % (size, size, h, w))
+        out = torch.empty((n, ca + cb, size, size), device=a.device, dtype=torch.float32)
+        with _on(a):
+            _ck(L.lib().v2v_crop_concat_forward(_p(a), ca, _p(b), cb, n, h, w, _p(win), size, size, _p(out), _st(a)))
+        ctx.save_for_backward(win)
+        ctx.dims = (ca, cb, n, h, w, size)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        if not ctx.needs_input_grad[1]:
+            return None, None, None, None
+        (win,) = ctx.saved_tensors
+        ca, cb, n, h, w, size = ctx.dims
+        g = g.contiguous()
+        gb = torch.empty((n, cb, h, w), device=g.device, dtype=torch.float32)
+        _ck(L.lib().v2v_crop_backward(_p(g), ca, cb, n, h, w, _p(win), size, size, _p(gb), L.current_stream_ptr()))
+        return None, gb, None, None
+
+
+def crop_concat(a, b, win, size):
+    """The face discriminator's input (vid2vid_model_D.py:152-153 + compute_loss_D's cat): (N, Ca+Cb, size, size)."""
+    return CropConcatFunction.apply(a, b, win, size)

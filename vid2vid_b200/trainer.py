@@ -1,6 +1,7 @@
 """The training step of train.py:50-93 on the B200 engine, one process per GPU.
 
-  * `FlatGrads`: every parameter's .grad is a view into ONE flat fp32 buffer laid out [G | D | D_T0 | ...]; a step issues a
+  * `FlatGrads`: every parameter's .grad is a view into ONE flat fp32 buffer laid out [G | D | D_T0 | ...] (D holds netD and,
+    with --add_face_disc, netD_f: the two share optimizer_D as in vid2vid_model_D.py:76-85); a step issues a
     single NCCL all-reduce(SUM) / world over it (SURVEY 8e) -- the replacement of DataParallel's per-forward parameter
     broadcast + per-backward reduce-to-GPU-0 (models/models.py:10-59).  Batch statistics stay per rank, as under DataParallel.
   * `Trainer.step`: generator forward (Vid2VidModelG.forward), reference flow (FlowNet, no grad), image / temporal
@@ -91,8 +92,10 @@ class Trainer:
     def __init__(self, opt, modelG, modelD, flowNet, world=1):
         self.opt, self.modelG, self.modelD, self.flowNet, self.world = opt, modelG, modelD, flowNet, world
         self.tG, self.tD, self.t_scales = opt.n_frames_G, opt.n_frames_D, opt.n_scales_temporal
-        groups = [[p for s in range(modelG.n_scales) for p in getattr(modelG, 'netG' + str(s)).parameters()],
-                  list(modelD.netD.parameters())]
+        params_D = list(modelD.netD.parameters())
+        if getattr(modelD, 'add_face_disc', False):
+            params_D += list(modelD.netD_f.parameters())     # each rank's window comes from its own shard, as per replica
+        groups = [[p for s in range(modelG.n_scales) for p in getattr(modelG, 'netG' + str(s)).parameters()], params_D]
         groups += [list(getattr(modelD, 'netD_T' + str(s)).parameters()) for s in range(self.t_scales)]
         self.grads = FlatGrads(groups)
         self.reset_clip()

@@ -85,3 +85,31 @@ def synth_label_sequence(n_frames, H, W, label_nc=35, block=8, seed=0, drift=1):
         m = m.repeat_interleave(block, 0).repeat_interleave(block, 1)[:H, :W]
         frames.append(m)
     return torch.stack(frames).float().view(1, n_frames, 1, H, W)
+
+
+def synth_pose_sequence(n_frames, H, W, seed=0, block=8, face=True, openpose=False, face_size=6, face_yx=None, drift=1):
+    """Synthetic pose-style input clip (label_nc 0, input_nc 6): U(-1,1) blobs on a zero background -- each coarse cell of a
+    block-pixel grid carries one with probability 0.3, drifting `drift` cells per frame -- plus a `face_size`-pixel "face"
+    patch drifting one pixel per frame from `face_yx` (default: a seeded interior position).  The face is channel 2 = 0.95,
+    or with `openpose` the openpose face colour (0.2, -1, -0.6) in channels 0-2; these are what the face detector of
+    Vid2VidModelD.get_face_region looks for, so blob values in channel 2 are capped at 0.85 to keep them out of it.
+    Returns float tensor (1, n_frames, 6, H, W)."""
+    g = torch.Generator().manual_seed(seed)
+    gh, gw = (H + block - 1) // block, (W + block - 1) // block
+    vals = torch.rand(6, gh, gw + drift * n_frames, generator=g) * 2 - 1
+    vals = vals * (torch.rand(1, gh, gw + drift * n_frames, generator=g) < 0.3).float()
+    vals[2].clamp_(max=0.85)
+    if face_yx is None:
+        face_yx = (int(torch.randint(0, max(1, H - face_size - n_frames), (1,), generator=g)),
+                   int(torch.randint(0, max(1, W - face_size - n_frames), (1,), generator=g)))
+    colour = (0.2, -1.0, -0.6) if openpose else (None, None, 0.95)
+    frames = []
+    for t in range(n_frames):
+        f = vals[:, :, t * drift: t * drift + gw].repeat_interleave(block, 1).repeat_interleave(block, 2)[:, :H, :W].clone()
+        if face:
+            y0, x0 = min(face_yx[0] + t, H - face_size), min(face_yx[1] + t, W - face_size)
+            for c, v in enumerate(colour):
+                if v is not None:
+                    f[c, y0:y0 + face_size, x0:x0 + face_size] = v
+        frames.append(f)
+    return torch.stack(frames).view(1, n_frames, 6, H, W)
